@@ -31,6 +31,7 @@ import json
 import os
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
@@ -42,6 +43,7 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 METRIC = "particle-RK4-steps/sec"
+DUMP_BYTES = 60 << 20  # --dump-outputs: all files of one run together stay below 64 MB
 _G = {}
 
 
@@ -322,6 +324,24 @@ class ClockSampler:
         reasons = [n for i, n in enumerate(names) if any(s[2 + i].lower().startswith("active") for s in self.samples)]
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(mx) if mx else None, "reasons": reasons,
                 "samples": len(self.samples)}  # fmt: skip
+
+
+def dump_outputs(out_dir, name, d, input_ids, max_bytes):
+    """Write the particle set ``d`` as ParticleSet.execute hands it back (deleted particles dropped, order kept) to
+    ``out_dir/<name>_<variable>.npy``.  Integer variables are stored as float64 (exact below 2**53).  If the set is larger than
+    ``max_bytes``, only the survivors of a fixed seeded sample of the released particles (``input_ids``) are written, so that two
+    builds write the same rows wherever they agree on which particles survive."""
+    from parcels_b200.statuscodes import StatusCode
+
+    rows = np.flatnonzero(d["state"] != StatusCode.Delete)
+    m = max_bytes // (8 * sum(int(np.prod(v.shape[1:])) for v in d.values()))  # (at most 8 bytes a value)
+    if len(rows) > m:
+        sample = input_ids[np.random.default_rng(0).choice(len(input_ids), size=min(m, len(input_ids)), replace=False)]
+        rows = rows[np.isin(d["particle_id"][rows], sample)]
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in d.items():
+        v = v[rows]
+        np.save(os.path.join(out_dir, f"{name}_{k}.npy"), v if v.dtype.kind == "f" else v.astype(np.float64))
 
 
 def measured_peak():
@@ -607,39 +627,47 @@ def run_gpu_workload(a, name, *, rank, local_rank, world, dist, steps, warmup, w
     value = total_steps / (dev_ms * 1e-3)
     kernel_ms = ksum / steps
     steps_per_launch = psteps / steps
+    if a.dump_outputs and rank == 0:
+        last = eng.download_all(ngrids=len(fs.gridset))
+        last["dt"][:] = dt
+        dump_outputs(a.dump_outputs, name, last, init["particle_id"], a.dump_bytes)
+        del last
 
     # ---- end-to-end arm: public API with host arrays; H2D + D2H of the particle SoA every step ----
     e2e = None
     if with_e2e:
-        k_e2e = min(steps, 5) if n_per_gpu > 2_000_000 else steps
+        k_e2e = steps
+        # one page-locked host input batch (inputs come from pinned host memory), refilled from `init` before every pass, outside
+        # the timed region
+        batch = {k: torch.from_numpy(np.ascontiguousarray(v)).pin_memory().numpy() for k, v in init.items()}
 
-        def pinned(v):  # page-locked host copy (the contract's "inputs from pinned host memory")
-            return torch.from_numpy(np.ascontiguousarray(v)).pin_memory().numpy()
-
-        fresh = [{k: pinned(v) for k, v in init.items()} for _ in range(k_e2e)]  # host input batches, made before timing
-        if a.pipeline >= 0:
-            ps.pipeline_chunks = a.pipeline
-        ps.eager_host = True  # this arm reads the result on the host after every pass: the download belongs to the (pipelined) call
-        for _ in range(min(warmup, 2)):
-            ps._data = {k: pinned(v) for k, v in init.items()}
-            ps.execute(kernels, dt=dt, runtime=runtime)
-            _ = ps._data
-        barrier()
-        e2e_steps = 0
-        t0 = time.perf_counter()
-        for i in range(k_e2e):
-            ps._data = fresh[i]
+        def e2e_pass():
+            for k, v in init.items():
+                np.copyto(batch[k], v)
+            ps._data = dict(batch)  # (execute leaves shortened views of these arrays in ps._data when particles are deleted)
+            barrier()
+            t0 = time.perf_counter()
             ps.execute(kernels, dt=dt, runtime=runtime)
             result = ps._data  # device -> host read of the step's result (the particle SoA after the pass)
             assert not ps._host_stale and len(result["x"]) > 0
+            barrier()
+            return time.perf_counter() - t0
+
+        if a.pipeline >= 0:
+            ps.pipeline_chunks = a.pipeline
+        ps.eager_host = True  # this arm reads the result on the host after every pass: the download belongs to the (pipelined) call
+        for _ in range(warmup):
+            e2e_pass()
+        e2e_steps, e2e_s = 0, 0.0
+        for _ in range(k_e2e):
+            e2e_s += e2e_pass()
             e2e_steps += ps.last_report["particle_steps"]
-        barrier()
-        e2e_s = reduce(time.perf_counter() - t0, "MAX")
+        e2e_s = reduce(e2e_s, "MAX")
         n = n_per_gpu
         e2e = {"value": reduce(e2e_steps, "SUM") / e2e_s, "unit": "particle-steps/s", "h2d_bytes_per_step": n * (6 * 4 + 8 + 4 + 4 + 8),
                "d2h_bytes_per_step": n * (6 * 4 + 8 + 4 + 4), "steps": k_e2e, "pipeline_chunks": ps.pipeline_chunks, "eager_host": True,
                "api": f"parcels_b200.ParticleSet.execute([{', '.join(w['kernels'])}, DeleteParticle], dt={dt:g}, runtime={runtime:g})"}  # fmt: skip
-        del fresh
+        del batch
 
     out = None
     if rank == 0:
@@ -723,7 +751,7 @@ def run_decomposed_bench(a, rank, local_rank, world, dist, workload="c5"):
     runtime = dt * nsteps
     kernels = [pb.AdvectionRK4_3D, pb.DeleteParticle]
     dev = f"cuda:{local_rank}"
-    steps, warmup = min(a.steps, 5), min(a.warmup, 2)
+    steps, warmup = a.steps, a.warmup
 
     eng = dfs.engine
     plan = D.decomposed_plan(dfs, kernels)
@@ -762,15 +790,15 @@ def run_decomposed_bench(a, rank, local_rank, world, dist, workload="c5"):
     n_after = D.allreduce_sum(eng.particle_count(), dist, dev)
 
     # ---- end-to-end arm: host particle arrays in, host arrays out (upload + rounds + download inside the timed region) ----
-    k_e2e = min(steps, 3)
+    k_e2e = steps
     e_t, e_steps = 0.0, 0
-    for i in range(k_e2e + 1):
+    for i in range(warmup + k_e2e):
         pdata = fresh()
         sync_all()
         t0 = time.perf_counter()
         out, stats = D.execute_decomposed(dfs, pdata, kernels, dt, runtime, dist)
         sync_all()
-        if i > 0:  # (the first one warms up)
+        if i >= warmup:
             e_t += D.allreduce_max(time.perf_counter() - t0, dist, dev)
             e_steps += D.allreduce_sum(stats["particle_steps"], dist, dev)
     fs.release()
@@ -863,6 +891,10 @@ def main():
     ap.add_argument("--sorted", action="store_true",
                     help="experiment: release the particles ordered by grid cell (z, y, x) instead of randomly -- measures what "
                          "spatial coherence between the lanes of a warp is worth (DESIGN.md 4, 'why not Morton-sort')")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the particle arrays the last device-resident pass of every workload of the line "
+                         "left (rank 0) as DIR/<workload>_<variable>.npy, float32 / float64, a fixed sample of particles where the "
+                         f"whole set would exceed {DUMP_BYTES >> 20} MB in all")
     a = ap.parse_args()
 
     rank = int(os.environ.get("RANK", "0"))
@@ -882,9 +914,16 @@ def main():
 
     import torch
 
-    from parcels_b200 import build
+    from oracle import c_port
+    from parcels_b200 import _lib, build
 
-    build.build()
+    # the tree may be read-only: a library older than its sources is compiled into a temporary directory, never into the tree
+    tmp = None
+    if build.needs_build():
+        tmp = tempfile.mkdtemp(prefix="parcels_b200_bench_")
+        _lib.LIB_PATH = build.build(out=os.path.join(tmp, "libparcels_b200.so"))
+    if c_port.needs_build():
+        c_port.LIB = os.path.join(tmp or tempfile.mkdtemp(prefix="parcels_b200_bench_"), "liboracle_c.so")
     dist = None
     if world > 1:
         import torch.distributed as dist
@@ -913,14 +952,16 @@ def main():
     w = WORKLOADS[name]
     extras = a.extras.split(",") if a.extras else (["c2", "c3", "c4"] if (name == "ns" and world == 1 and a.extras is None) else [])
     extras = [e for e in extras if e and e != name]
+    if a.dump_outputs:
+        a.dump_bytes = DUMP_BYTES // (1 + len(extras))  # an equal share of the budget for every workload of the line
     cache = {}
     t_main = time.perf_counter()
     main_out = run_gpu_workload(a, name, rank=rank, local_rank=local_rank, world=world, dist=dist, steps=a.steps, warmup=a.warmup,
                                 with_e2e=not a.no_e2e, with_cpu=not a.no_cpu_baseline, field_cache=cache)  # fmt: skip
     extra_out = {}
     for e in extras:
-        r = run_gpu_workload(a, e, rank=rank, local_rank=local_rank, world=world, dist=dist, steps=max(3, min(a.steps, 5)),
-                             warmup=max(3, min(a.warmup, 3)), with_e2e=not a.no_e2e, with_cpu=not a.no_cpu_baseline, field_cache=cache)  # fmt: skip
+        r = run_gpu_workload(a, e, rank=rank, local_rank=local_rank, world=world, dist=dist, steps=a.steps, warmup=a.warmup,
+                             with_e2e=not a.no_e2e, with_cpu=not a.no_cpu_baseline, field_cache=cache)  # fmt: skip
         if r is not None:
             r["config"] = config_block(e, WORKLOADS[e], a.particles or WORKLOADS[e]["n"])
             extra_out[e] = r

@@ -20,10 +20,14 @@ class _Grid(C.Structure):
                 ("U", C.c_void_p), ("V", C.c_void_p), ("W", C.c_void_p)]  # fmt: skip
 
 
+def needs_build():
+    return not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(os.path.join(HERE, "advect_rk4_3d.c"))
+
+
 def build():
-    src = os.path.join(HERE, "advect_rk4_3d.c")
-    if not os.path.exists(LIB) or os.path.getmtime(LIB) < os.path.getmtime(src):
-        subprocess.run(["make", "-C", HERE, "-B", "_build/liboracle_c.so"], check=True, capture_output=True)
+    """Compile to ``LIB`` (set it to a path outside the tree to build there)."""
+    if needs_build():
+        subprocess.run(["make", "-C", HERE, "-B", f"LIB={LIB}", LIB], check=True, capture_output=True)
     return LIB
 
 

@@ -315,6 +315,80 @@ def make_output_golden():
     np.savez_compressed(os.path.join(GOLDEN, "output_rows.npz"), **out)
 
 
+def make_output_rule_random_golden():
+    """The reference's ``_to_write_particles`` on 20 seeded random draws (tests/test_output_cpu.py)."""
+    from oracle import ref_harness as rh
+
+    rh.install()
+    from parcels._core.particlefile import _to_write_particles
+
+    out = {}
+    rng = np.random.default_rng(5)
+    for k in range(20):
+        n = 500
+        t = np.round(rng.uniform(0, 100, n))
+        t[rng.uniform(size=n) < 0.1] = np.nan
+        dt = np.full(n, rng.choice([-7.0, 3.0, 10.0]))
+        tout = float(np.round(rng.uniform(0, 100)))
+        out[f"t{k}"], out[f"dt{k}"], out[f"tout{k}"] = t, dt, np.array(tout)
+        out[f"rows{k}"] = _to_write_particles({"t": t, "dt": dt, "particle_id": np.arange(n)}, tout)
+    np.savez_compressed(os.path.join(GOLDEN, "output_rule_random.npz"), **out)
+
+
+def _fieldset_record(fs):
+    """What ``parcels_b200.adapter.from_parcels`` reads from a reference FieldSet, as plain values (tests/test_adapter_cpu.py
+    rebuilds the object from it)."""
+    g = fs.U.grid
+    md = g.sgrid_metadata
+
+    def pad(p):
+        return str(getattr(p, "value", p))
+
+    axes = list(g.axes)
+    return {
+        "grid": {"axes": axes, "xdim": int(g.xdim), "ydim": int(g.ydim), "zdim": int(g.zdim) if "Z" in axes else None,
+                 "deg2m": float(g.deg2m), "spherical": bool(g._mesh.is_spherical()), "radius": getattr(g._mesh, "radius", None),
+                 "padding": [pad(f.padding) for f in md.face_dimensions],
+                 "vertical_padding": [pad(v.padding) for v in md.vertical_dimensions] if md.vertical_dimensions else None},
+        "time_ns": None if fs.U.time_interval is None else np.asarray(fs.U.data.time.values).astype(np.int64).tolist(),
+        "fields": {name: {"interp": type(getattr(f, "interp_method", None)).__name__, "on_grid": getattr(f, "grid", None) is g,
+                          "spherical": bool(f.grid._mesh.is_spherical()) if hasattr(f, "grid") else None}
+                   for name, f in fs.fields.items()},
+        "vector": type((getattr(fs, "UVW", None) or fs.UV).interp_method).__name__,
+        "gridset": len(fs.gridset),
+        "context": dict(fs.context),
+    }  # fmt: skip
+
+
+def make_adapter_golden():
+    """Reference FieldSets / a ParticleSet as ``parcels_b200.adapter`` sees them (tests/test_adapter_cpu.py)."""
+    import cases as tc
+    from oracle import ref_harness as rh
+
+    def fieldset(c, **kw):
+        return rh.build_fieldset(lon=c["lon"], lat=c["lat"], depth=c["depth"], times=c["times"], U=c["U"], V=c["V"], W=c["W"],
+                                 mesh=c["mesh"], **kw)  # fmt: skip
+
+    rec, out = {}, {}
+    c = tc.build(tc.CASES["diffusion"])
+    ref = fieldset(c, constants=c["constants"])
+    rec["diffusion"] = _fieldset_record(ref)
+    for k, v in rh.make_pset(ref, x=c["x"], y=c["y"], z=c["z"], t=c["t"])._data.items():
+        out[f"diffusion/pset/{k}"] = v
+    c = tc.build(tc.CASES["curv_sph_2d"])
+    rec["curv_sph_2d"] = _fieldset_record(fieldset(c, interp="cgrid_velocity", padding=c["padding"]))
+    c = tc.build(tc.CASES["flat_f32c_f64d"])
+    kz = np.abs(c["U"]) + 1
+    c["W"] = None
+    ref = fieldset(c, scalars={"Kh_zonal": (kz, "linear"), "Kh_meridional": (kz[:1], "linear")})
+    ref.add_context("dres", 12.5)
+    rec["flat_f32c_f64d"] = _fieldset_record(ref)
+    k = rh.kernels()
+    rec["kernel_modules"] = {name: getattr(k, name).__module__ for name in ("AdvectionDiffusionM1", "AdvectionRK4")}
+    out["record"] = np.array(json.dumps(rec))
+    np.savez_compressed(os.path.join(GOLDEN, "adapter_reference.npz"), **out)
+
+
 SCALAR_CASES = ("c2_small", "flat_f32c_f64d", "all_f32", "cgrid_rect_3d")
 
 
@@ -568,6 +642,8 @@ if __name__ == "__main__":
     make_v3("nearest", "v3_jit_nearest.npz")
     make_ref_cases()
     make_output_golden()
+    make_output_rule_random_golden()
+    make_adapter_golden()
     make_scalar_golden()
     make_scalar_curv_golden()
     make_rk45_golden()

@@ -7,8 +7,8 @@ registering permissive stub modules and a NumPy duck type for ``xarray.DataArray
 
 * ``oracle/make_golden.py`` -- generate the committed fixtures under ``tests/golden/``
   (outputs of the reference itself on seeded inputs);
-* ``tests/test_oracle_vs_reference.py`` -- when ``/root/reference`` is present, check the
-  NumPy restatement in ``oracle/parcels_oracle.py`` against the reference's own code.
+* ``tests/test_install_cpu.py`` -- where the reference package is present, run its own
+  ``ParticleSet.execute`` with and without ``parcels_b200.install()``.
 
 ``/root/reference`` does not exist on the GPU box: nothing reachable from ``-m gpu`` tests,
 ``smoke()`` or ``bench.py`` imports this file.

@@ -26,19 +26,20 @@ NVCC_FLAGS = [
 ]  # fmt: skip
 
 
-def needs_build() -> bool:
-    if not os.path.exists(OUT):
+def needs_build(out: str = OUT) -> bool:
+    if not os.path.exists(out):
         return True
-    t = os.path.getmtime(OUT)
+    t = os.path.getmtime(out)
     return any(os.path.getmtime(f) > t for f in (*DEPS, HEADER, __file__))
 
 
-def build(force: bool = False, verbose: bool = False) -> str:
-    if not force and not needs_build():
-        return OUT
-    os.makedirs(os.path.dirname(OUT), exist_ok=True)
+def build(force: bool = False, verbose: bool = False, out: str = OUT) -> str:
+    """Compile the library to ``out`` (object files go to ``obj/`` beside it); returns ``out``."""
+    if not force and not needs_build(out):
+        return out
+    os.makedirs(os.path.dirname(out), exist_ok=True)
     nvcc = os.environ.get("NVCC", "nvcc")
-    objdir = os.path.join(HERE, "lib", "obj")
+    objdir = os.path.join(os.path.dirname(out), "obj")
     os.makedirs(objdir, exist_ok=True)
     procs = []
     for src in SOURCES:
@@ -48,17 +49,17 @@ def build(force: bool = False, verbose: bool = False) -> str:
         procs.append((cmd, obj, subprocess.Popen(cmd, stdout=subprocess.PIPE, stderr=subprocess.PIPE, text=True)))
     objs = []
     for cmd, obj, p in procs:
-        out, err = p.communicate()
+        stdout, err = p.communicate()
         if p.returncode != 0:
-            raise RuntimeError(f"nvcc failed:\n{' '.join(cmd)}\n{out}\n{err}")
+            raise RuntimeError(f"nvcc failed:\n{' '.join(cmd)}\n{stdout}\n{err}")
         if verbose:
             print(err)
         objs.append(obj)
-    cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", OUT, *objs, "-ldl"]
+    cmd = [nvcc, "-shared", "-gencode", "arch=compute_100a,code=sm_100a", "-o", out, *objs, "-ldl"]
     res = subprocess.run(cmd, capture_output=True, text=True)
     if res.returncode != 0:
         raise RuntimeError(f"link failed:\n{' '.join(cmd)}\n{res.stdout}\n{res.stderr}")
-    return OUT
+    return out
 
 
 if __name__ == "__main__":

@@ -1,36 +1,18 @@
-"""CPU test (build container only): the oracle restatement is bit-identical to the reference's
-own code, imported from /root/reference through oracle/ref_harness.py.  Skipped where the
-reference tree is absent (e.g. on the GPU box)."""
+"""CPU test: the oracle restatement is bit-identical to the reference's own code, run on the same cases
+through ParticleSet.execute with its own kernels and a user DeleteParticle handler.  The reference's
+outputs are stored in tests/golden/ref_cases.npz (oracle/make_golden.py)."""
+
+import os
 
 import numpy as np
 import pytest
 
-import cases
-from oracle import ref_harness as rh
 from oracle_run import load_case, run_oracle
-
-pytestmark = pytest.mark.skipif(not rh.reference_available(), reason="/root/reference not present")
 
 
 @pytest.mark.parametrize("name", ["c2_small", "all_f32", "delayed_partial", "diffusion", "raise_oob"])
-def test_live_reference_equals_oracle(name):
-    c = load_case(name)
-    fs = rh.build_fieldset(lon=c["lon"], lat=c["lat"], depth=c["depth"], times=c["times"], U=c["U"], V=c["V"],
-                           W=c["W"], mesh=c["mesh"], constants=c["constants"])  # fmt: skip
-    ps = rh.make_pset(fs, x=c["x"], y=c["y"], z=c["z"], t=c["t"])
-    k = rh.kernels()
-
-    def DeleteParticle(particles, fieldset):
-        particles[particles.state >= 50].state = 30
-
-    kern = [getattr(k, kn) for kn in c["kernels"]] + ([DeleteParticle] if c["delete_on_error"] else [])
-    if c["rng_seed"] is not None:
-        np.random.seed(c["rng_seed"])
-    try:
-        for seg in c["segments"]:
-            ps.execute(kern, dt=c["dt"], verbose_progress=False, **seg)
-    except RuntimeError:
-        pass
-    pd, _ = run_oracle(c)
+def test_live_reference_equals_oracle(name, golden_dir):
+    ref = np.load(os.path.join(golden_dir, "ref_cases.npz"))
+    pd, _ = run_oracle(load_case(name))
     for key in ("particle_id", "state", "ei", "t", "x", "y", "z"):
-        np.testing.assert_array_equal(ps._data[key], pd[key], err_msg=key)
+        np.testing.assert_array_equal(ref[f"{name}/{key}"], pd[key], err_msg=key)

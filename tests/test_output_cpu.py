@@ -29,22 +29,13 @@ def test_selection_rule_matches_reference_outputs(golden_dir):
 
 
 def test_selection_rule_matches_reference_code(golden_dir):
-    from oracle import ref_harness as rh
-
-    if not rh.reference_available():
-        pytest.skip("reference tree not mounted")
-    rh.install()
-    from parcels._core.particlefile import _to_write_particles
-
-    rng = np.random.default_rng(5)
-    for _ in range(20):
-        n = 500
-        t = np.round(rng.uniform(0, 100, n))
-        t[rng.uniform(size=n) < 0.1] = np.nan
-        d = {"t": t, "dt": np.full(n, rng.choice([-7.0, 3.0, 10.0])), "particle_id": np.arange(n)}
-        tout = float(np.round(rng.uniform(0, 100)))
-        np.testing.assert_array_equal(po.to_write_particles(d, tout), _to_write_particles(d, tout))
-        np.testing.assert_array_equal(to_write_particles(d, tout), _to_write_particles(d, tout))
+    """20 random draws and the rows the reference's own _to_write_particles selected for them (oracle/make_golden.py)."""
+    g = np.load(os.path.join(golden_dir, "output_rule_random.npz"))
+    for k in range(20):
+        d = {"t": g[f"t{k}"], "dt": g[f"dt{k}"], "particle_id": np.arange(len(g[f"t{k}"]))}
+        tout = float(g[f"tout{k}"])
+        np.testing.assert_array_equal(po.to_write_particles(d, tout), g[f"rows{k}"])
+        np.testing.assert_array_equal(to_write_particles(d, tout), g[f"rows{k}"])
 
 
 def _tiny_pset(n=50, pclass=pb.Particle, **kw):
